@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py -- the driver's benchmark contract for carla_ppo_b200.
+"""bench.py -- the benchmark of carla_ppo_b200.
 
     python bench.py --gpus N --steps K --warmup W            (this build: sm_100a CUDA behind the C ABI)
+    python bench.py --steps K --warmup W --dump-outputs DIR  (also write what the last timed step computed, see below)
     python bench.py --impl reference --steps K --warmup W    (the reference's CPU path on the host cores)
     python bench.py --config 5 [--gpus N]                    (BASELINE configs[4]: 100 k frames -> encode -> PPO loop)
 
@@ -21,6 +22,13 @@ One JSON line on stdout (rank 0).  Keys follow the contract:
                peaks are measured here, BASELINE.md section 3) + per-group device times on rank 0 (also for N>1);
   dp_check     (N>1) replicas bit-identical after the timed steps, N-rank loss / gradient vs a 1-rank recompute;
   cpu_baseline torch-CPU fp32 restatement of the reference graph ("port": TensorFlow 1.13 cannot be installed).
+
+--steps K is the number of steps of every timed loop (device-resident, host-fed, blocking host entry, PPO learn()).
+--dump-outputs DIR (rank 0) writes, as DIR/<name>.npy in float32, what a caller of each timed path holds after its last
+timed call: vae_losses ([recon, kl] the step returns), vae_params.<tensor> (the parameters it updated in place) and
+vae_grads.<tensor> (the gradient that update used); ppo_metrics (the per-minibatch losses of the last learn()) and
+ppo_params.<tensor> (N=1 only).  Tensor names are the reference's variable names with '/' -> '.'.  The inputs and
+weights are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import ctypes as C
@@ -46,6 +54,24 @@ BYTES_PER_FRAME_TRAIN = 10_164_000           # layer-materialised fp32 model, SU
 MAC = {"conv1": 4_732_416, "conv2": 22_413_312, "conv3": 18_874_368, "conv4": 12_582_912,
        "heads": 786_432, "dense1": 393_216, "deconv1": 12_582_912, "deconv2": 18_874_368,
        "deconv3": 35_020_800, "deconv4": 4_732_416}
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def tensor_dumps(prefix, tensors):
+    """{'<prefix>.<name with / -> .>': float32 array} of a name -> array dict (get_weights() / get_grads())."""
+    return {"%s.%s" % (prefix, k.replace("/", ".")): np.asarray(v, np.float32) for k, v in tensors.items()}
+
+
+def write_dumps(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy, refusing a set larger than DUMP_LIMIT_BYTES."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def kernel_source_hash():
@@ -211,9 +237,10 @@ def shipped_agent():
             {k: z["adam_v/" + k] for k in names}, (float(z["beta1_power"]), float(z["beta2_power"])))
 
 
-def bench_ppo(lib, steps=10, cpu=True):
+def bench_ppo(lib, steps=10, cpu=True, dumps=None):
     """BASELINE configs[2]: T=2048 rollout of 67-d states, 4 epochs x 8 minibatches of 256, weights = the reference's shipped
-    agent checkpoint-705 (policy, policy_old, warm Adam slots); timed: GAE + normalisation + theta_old copy + 32 Adam steps."""
+    agent checkpoint-705 (policy, policy_old, warm Adam slots); timed: GAE + normalisation + theta_old copy + 32 Adam steps.
+    `dumps` (a dict) receives the metrics and parameters of the last timed learn()."""
     import torch
     from carla_ppo_b200.ppo import PPO
 
@@ -239,6 +266,9 @@ def bench_ppo(lib, steps=10, cpu=True):
     for _ in range(steps):
         ppo.learn(s, a, v, r, d, 0.3, num_epochs=E, batch_size=B, perms=perms)
     e1.record(); torch.cuda.synchronize()
+    if dumps is not None:
+        dumps["ppo_metrics"] = ppo._pending_metrics[-1].cpu().numpy()
+        dumps.update(tensor_dumps("ppo_params", ppo.get_weights()))
     ms = e0.elapsed_time(e1) / steps
     launches = int(lib.cpb_launch_count()) // steps
     out = {"metric": "PPO latent-updates/sec", "value": T * E / ms * 1e3, "unit": "sample-updates/s", "ms_per_learn": ms,
@@ -360,6 +390,12 @@ def run_ours(args):
         vae.train_step_device(x, x, eps)
     e1.record()
     barrier()
+    dumps = None
+    if args.dump_outputs and rank == 0:
+        # copied before anything else runs: the e2e and profiling steps below keep training the same model
+        dumps = {"vae_losses": vae._losses.cpu().numpy()}
+        dumps.update(tensor_dumps("vae_params", vae.get_weights()))
+        dumps.update(tensor_dumps("vae_grads", vae.get_grads()))
     launches = int(lib.cpb_launch_count())
     elapsed = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -384,7 +420,7 @@ def run_ours(args):
                 pending.result()
             pending = h
         pending.result()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     e2e_run(2); barrier()
     t0 = time.perf_counter()
     e2e_run(e2e_steps)
@@ -484,7 +520,7 @@ def run_ours(args):
                                  "frac": BYTES_PER_FRAME_TRAIN * GLOBAL_BATCH / (ms_step * 1e-3) / 1e9 / peaks["hbm_gbs"]},
                     "groups_ms_per_step": {k: round(v["ms_per_step"], 4) for k, v in sorted(groups.items(), key=lambda kv: -kv[1]["ms_per_step"])}}
         cpu = cpu_baseline_vae() if (world == 1 and not args.no_cpu_baseline) else None
-        ppo = bench_ppo(lib, cpu=not args.no_cpu_baseline) if world == 1 else None
+        ppo = bench_ppo(lib, steps=args.steps, cpu=not args.no_cpu_baseline, dumps=dumps) if world == 1 else None
         out = {"metric": "VAE frames/sec @ batch 4096", "value": value, "unit": "frames/s", "n_gpus": world,
                "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": ms_step, "higher_is_better": True,
                "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -507,6 +543,8 @@ def run_ours(args):
             out["cpu_baseline"] = cpu
         if ppo:
             out["ppo"] = ppo
+        if dumps is not None:
+            write_dumps(args.dump_outputs, dumps)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -563,7 +601,13 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 5],
                     help="2 (default): the BASELINE metric, ConvVAE train step at batch 4096; 5: BASELINE configs[4], the offline "
                          "100k-frame encode -> PPO update pipeline (scripts/config5.py; frames sharded over the ranks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 2 or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the default benchmark (--impl ours --config 2)")
     if args.config == 5:
         import runpy
         sys.argv = [os.path.join(ROOT, "scripts", "config5.py")]
